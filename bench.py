@@ -19,6 +19,8 @@ line carries the other vocabularies / hit rates / rule counts as extra.variants.
 `--impl reference` times the reference path's CPU restatement (Node.js is not in this image or on
 the GPU box, and the reference has no native sources to compile, so oracle/ is the only runnable
 form of it) on all host threads.
+`--dump-outputs DIR` writes the result words of the last timed step (rank 0) to DIR/scan_words.npy: the inputs are seeded,
+so two builds of the project run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -42,6 +44,21 @@ C4_MSGS = 10_000_000
 MERKLE_LEAVES = 1 << 24
 MERKLE_LEAF = 256
 MERKLE_BLOCK_LOG2 = 16
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_scan_words(out_dir, words):
+    """--dump-outputs: the result words a caller of the timed path receives (uint64 per message: hit << 63 |
+    #rules hit << 32 | lowest hit rule) as DIR/scan_words.npy, float64 [k, 3] = (message index, high 32 bits, low 32
+    bits), exact in float64.  Batches whose rows exceed DUMP_MAX_BYTES are sampled at fixed, seeded message indices."""
+    words = np.ascontiguousarray(words).view(np.uint64)
+    n = len(words)
+    cap = (DUMP_MAX_BYTES - 4096) // (3 * 8)
+    idx = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    w = words[idx]
+    table = np.stack([idx.astype(np.float64), (w >> np.uint64(32)).astype(np.float64), (w & np.uint64(0xFFFFFFFF)).astype(np.float64)], axis=1)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scan_words.npy"), table)
 
 
 def measured_peaks():
@@ -155,8 +172,10 @@ def reference_arm(args, rank, world, emit=None):
         O.scan_policy(regs, data, off, threads=threads, want_bits=False)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.scan_policy(regs, data, off, threads=threads, want_bits=False)
+        _, words = O.scan_policy(regs, data, off, threads=threads, want_bits=False)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_scan_words(args.dump_outputs, words)
     v = sample * args.steps / dt
     node = find_node()
     line = {"metric": "messages_scanned_per_s", "value": v, "unit": "msgs/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -201,7 +220,11 @@ def main():
     ap.add_argument("--no-variants", action="store_true")
     ap.add_argument("--no-c4", action="store_true")
     ap.add_argument("--merkle-leaves", type=int, default=MERKLE_LEAVES)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result words of the last one to DIR/scan_words.npy (see dump_scan_words)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global P_HIT
     if args.p_hit is not None:
         P_HIT = args.p_hit
@@ -237,7 +260,8 @@ def main():
         return d, o64.to(torch.int32), injected        # uint32 offsets (bit pattern) as the C ABI expects; n*L < 2^31 here
 
     def measure(ruleset, d, o, nmsgs, steps, warmup, profile_steps):
-        """-> (ms_per_step over `steps` graph-replayed steps, per-kernel ms medians, counters, result words of the last step)"""
+        """-> (ms_per_step over `steps` graph-replayed steps, per-kernel ms medians, counters, result words of the last timed step,
+        whether every timed step's words equal the profiled step's)"""
         outs = [torch.zeros(nmsgs, dtype=torch.int64, device=dev) for _ in range(2)]
         k = [0]
 
@@ -273,7 +297,7 @@ def main():
             ruleset.scan_join(stream.cuda_stream)        # waits for the stream; raises if a batch overflowed a queue
             torch.cuda.synchronize()
         same = bool(torch.equal(outs[0], ref_words) and torch.equal(outs[1], ref_words))
-        return e0.elapsed_time(e1) / steps, np.median(np.array(kms), axis=0), counters, ref_words, same
+        return e0.elapsed_time(e1) / steps, np.median(np.array(kms), axis=0), counters, outs[(k[0] - 1) & 1], same
 
     # ---- headline: K steps, device-resident inputs (256 MiB per step > 126 MB L2), barrier + sync both sides
     data, off, inj = gen(n, rl, P_HIT, args.seed_offset, args.vocab, args.frag_frac)
@@ -674,6 +698,8 @@ def main():
         "clocks": clocks,
         "extra": {"oracle_check": cpu if world > 1 else None, "variants": variants, "merkle": merkle, "c4": c4, "redact": redact, "scan_one": one, "per_rank_ms_per_step": per_rank_ms},
     }
+    if args.dump_outputs:
+        dump_scan_words(args.dump_outputs, words.cpu().numpy())
     emit(line)
     if world > 1:
         dist.destroy_process_group()
